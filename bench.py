@@ -54,7 +54,23 @@ def parse_args():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-graph", action="store_true", help="launch the step's kernels one by one instead of one CUDA graph")
     ap.add_argument("--cpu-budget-s", type=float, default=20.0, help="CPU baseline sample budget (seconds of queries)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed search step returned (ids, scores, minmax) and the last timed "
+                         "encode step's embeddings to DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """DIR/<name>.npy in float32 / float64 (int64 ids as float64, exact below 2**53), so that two builds run with the
+    same arguments -- hence the same seeded inputs -- can be compared output by output."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float32 if a.dtype == np.float32 else np.float64))
 
 
 def workload_config(rows: int, dim: int, nq: int, k: int, world: int) -> dict:
@@ -143,11 +159,10 @@ class ClockSampler:
 
 # ------------------------------------------------------------------------------------------ the reference's modules
 def find_reference_root():
-    """The reference checkout in the build container, or the unmodified copy tools/stage_reference.sh puts under
-    baseline/_ref (git-ignored, travels to the GPU box)."""
-    for cand in (os.environ.get("COMORAG_REFERENCE"), "/root/reference", os.path.join(ROOT, "baseline", "_ref")):
-        if cand and os.path.isdir(os.path.join(cand, "src", "comorag")):
-            return cand
+    """A ComoRAG checkout named by $COMORAG_REFERENCE, if any; without one the CPU arms time the oracle port."""
+    cand = os.environ.get("COMORAG_REFERENCE")
+    if cand and os.path.isdir(os.path.join(cand, "src", "comorag")):
+        return cand
     return None
 
 
@@ -534,6 +549,7 @@ def run_ours(args):
     value = args.nq / ms_per_step * 1e3
     got_ids = session.ids.clone()
     got_scores = session.scores.clone()
+    got_minmax = session.minmax.clone() if args.dump_outputs else None
     if index.peer is not None:
         index.peer.check()
 
@@ -626,7 +642,7 @@ def run_ours(args):
     # ---- encode (index build): data-parallel, every rank encodes its own batch
     encode = None
     if not args.no_encode:
-        encode = bench_encode(args, world, rank, dev, st, peaks, barrier, max_over_ranks)
+        encode, enc_out = bench_encode(args, world, rank, dev, st, peaks, barrier, max_over_ranks)
 
     # the sampler has been running through every GPU-timed phase above (search value, scan roofline, e2e, encode)
     clocks = sampler.stop() if rank == 0 else None
@@ -639,6 +655,13 @@ def run_ours(args):
                 encode["cpu_baseline"] = cpu_encode_baseline(ref, 64, args.encode_len)
             except Exception as e:  # transformers missing etc.: report, do not fake
                 encode["cpu_baseline"] = {"unavailable": repr(e)[:300]}
+
+    if rank == 0 and args.dump_outputs:
+        outputs = {"search_ids": got_ids.cpu().numpy(), "search_scores": got_scores.float().cpu().numpy(),
+                   "search_minmax": got_minmax.float().cpu().numpy()}
+        if encode is not None:
+            outputs["encode_embeddings"] = enc_out.cpu().numpy()
+        dump_outputs(args.dump_outputs, outputs)
 
     if rank == 0:
         if world == 1 or index.exchange_mode == "peer":
@@ -699,6 +722,7 @@ def bench_encode(args, world, rank, dev, st, peaks, barrier, max_over_ranks):
         enc.forward_packed(ids_dev, cu_dev, L, out_f32=out)
     b.record(st)
     barrier()
+    out_last = out.clone()      # the last timed encode step's embeddings (later phases reuse `out`)
     enc_ms = max_over_ranks(a.elapsed_time(b)) / args.encode_steps
     chunks_s = world * n / enc_ms * 1e3
     flops = cfg.flops_per_chunk(L) * n
@@ -780,7 +804,7 @@ def bench_encode(args, world, rank, dev, st, peaks, barrier, max_over_ranks):
             "probe_batch": {"probes": 32, "tokens_each": 24, "ms": probe_ms, "probes_per_s": 32 / probe_ms * 1e3,
                             "what": "encode_token_lists through the captured CUDA graph (768-token bucket), host call to result on device"},
             "tokenizer": tok,
-            "gpu_launches": args.encode_steps * launches_per_fwd}
+            "gpu_launches": args.encode_steps * launches_per_fwd}, out_last
 
 
 def main():

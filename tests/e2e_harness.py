@@ -9,8 +9,8 @@
 
 The same harness drives both arms -- the reference's own classes on CPU and the comorag_b200 shim on cuda:0 -- so
 whatever the stand-ins approximate, they approximate identically for both.  Nothing in here is product code; nothing
-in comorag_b200/ imports it.  The reference tree is looked up at $COMORAG_REFERENCE, /root/reference (build container)
-or <repo>/baseline/_ref (an unmodified copy staged by tools/stage_reference.sh, git-ignored, travels to the GPU box).
+in comorag_b200/ imports it.  Running the loop needs a reference checkout, named by $COMORAG_REFERENCE; the tests replay
+what such a run recorded (see "replay" below) and need no checkout.
 """
 from __future__ import annotations
 
@@ -30,10 +30,10 @@ CKPT = os.path.join(ROOT, "tests", "golden", "bge-tiny-synth")
 
 
 def find_reference_root() -> Optional[str]:
-    for cand in (os.environ.get("COMORAG_REFERENCE"), "/root/reference", os.path.join(ROOT, "baseline", "_ref")):
-        if cand and os.path.isdir(os.path.join(cand, "src", "comorag")) and \
-                os.path.isdir(os.path.join(cand, "dataset", "cinderella")):
-            return cand
+    cand = os.environ.get("COMORAG_REFERENCE")
+    if cand and os.path.isdir(os.path.join(cand, "src", "comorag")) and \
+            os.path.isdir(os.path.join(cand, "dataset", "cinderella")):
+        return cand
     return None
 
 
@@ -303,10 +303,12 @@ def _json_safe(x: Any) -> Any:
     return x
 
 
-def run_cinderella(arm: str, workdir: str, ref_root: str, max_loops: int = 1, questions: Optional[int] = None) -> Dict:
+def run_cinderella(arm: str, workdir: str, ref_root: str, max_loops: int = 1, questions: Optional[int] = None,
+                   capture=None) -> Dict:
     """arm = "reference": the reference's own classes on CPU (fp32 HF encoder, numpy search);
     arm = "shim": comorag_b200.install() first, then the SAME unmodified ComoRAG.py (needs cuda:0);
     arm = "shim_search": install(encoder=False): reference encoder, engine stores + device search (needs cuda:0).
+    `capture(rag, batch_encode)`, if given, runs after try_answer and its result is returned under "captured".
     Returns {"trace": {...}, "solutions": [...], "encodes": int, "kernel_search_calls": int}."""
     sys.dont_write_bytecode = True
     if ref_root not in sys.path:
@@ -433,6 +435,7 @@ def run_cinderella(arm: str, workdir: str, ref_root: str, max_loops: int = 1, qu
                 "timeline": rag.level_store.get_all_ids(),
             }
             n_edges = rag.graph.ecount()
+            captured = capture(rag, orig_be) if capture is not None else None
             wave = getattr(rag, "_crag_wave", None)
             wave_stats = dict(wave.stats) if wave is not None else None
             if wave is not None:
@@ -443,7 +446,8 @@ def run_cinderella(arm: str, workdir: str, ref_root: str, max_loops: int = 1, qu
         main.get_similar_summaries = orig_gss
     return {"arm": arm, "wave_stats": wave_stats if arm != "reference" else None, "trace": trace, "answers": [getattr(s, "answer", None) for s in solutions], "stores": stores,
             "graph_edges": n_edges, "index_encodes": index_encodes,
-            "query_encodes": {k: counters[k] - index_encodes[k] for k in counters}, "queries": queries}
+            "query_encodes": {k: counters[k] - index_encodes[k] for k in counters}, "queries": queries,
+            "captured": captured}
 
 
 # ------------------------------------------------------------------------------------------------ comparison
@@ -531,10 +535,143 @@ def compare_traces(ref: Dict, got: Dict, raw_tol: float = 4e-3, floor_tol: float
         if not ok:
             problems.append(f"{query!r} epi: {msg}")
         # what tri_retrieve hands to the memory pool (after the corpus-order re-sort): identical text lists
-        for part in ("veridical", "episodic", "semantic"):
+        for part in ("veridical", "episodic", "semantic") if "docs" in r else ():
             if sorted(r["docs"][part]) != sorted(g["docs"][part]):
                 problems.append(f"{query!r}: {part} docs differ")
         checked += 1
-    if ref["answers"] != got["answers"]:
+    if ref.get("answers") != got.get("answers"):
         problems.append("final answers differ")
     return {"queries": checked, "max_score_dev": worst, "max_ppr_dev": worst_ppr, "problems": problems}
+
+
+# ------------------------------------------------------------------------------------------------ replay
+# The reference tree is not part of this repository.  tests/golden/make_golden_e2e_replay.py ran the loop above on the
+# reference once and stored what its retrieval methods saw: every store's rows (texts, keys, the reference encoder's
+# fp32 embeddings) and every probe string with its query row.  Replaying those probes reproduces the fact / passage /
+# summary / timeline part of the committed trace without the reference.
+REPLAY = os.path.join(ROOT, "tests", "golden", "e2e_cinderella_replay.npz")
+STORE_NAMES = ("chunk", "entity", "fact", "summary", "timeline")
+REPLAYED_KINDS = ("fact_scores", "fact_range", "ver", "sem", "epi")
+
+
+def load_replay(path: str = REPLAY) -> Dict:
+    with np.load(path) as z:
+        rec = {k: z[k] for k in z.files}
+    rec["epi_top_k"] = int(rec["epi_top_k"])
+    return rec
+
+
+def retrieval_view(run: Dict) -> Dict:
+    """The stores and the REPLAYED_KINDS of every probe of a run (the part a replay can reproduce)."""
+    return {"stores": run["stores"],
+            "trace": {q: {k: v for k, v in t.items() if k in REPLAYED_KINDS} for q, t in run["trace"].items()}}
+
+
+def _entry(rec, q, facts, ver, sem, epi) -> Dict:
+    def rng(ns):
+        raw = rec[ns + "_emb"] @ np.asarray(q, dtype=np.float32).reshape(-1)
+        return float(raw.max() - raw.min())
+    keys = {ns: rec[ns + "_keys"].tolist() for ns in ("fact", "chunk", "summary")}
+    return {"fact_scores": dict(zip(keys["fact"], np.asarray(facts, dtype=np.float64).tolist())),
+            "fact_range": rng("fact"),
+            "ver": {"ids": [keys["chunk"][i] for i in np.asarray(ver[0]).tolist()],
+                    "scores": np.asarray(ver[1], dtype=np.float64).tolist(), "range": rng("chunk")},
+            "sem": {"ids": [keys["summary"][i] for i in np.asarray(sem[0]).tolist()],
+                    "scores": np.asarray(sem[1], dtype=np.float64).tolist(), "range": rng("summary")},
+            "epi": {"texts": [_h(t) for t in epi[0]], "scores": [float(s) for s in epi[1]], "range": rng("timeline")}}
+
+
+def replay_reference(rec: Dict) -> Dict:
+    """The reference's retrieval arithmetic (oracle/search_oracle.py restates it) on the recorded rows, on the CPU."""
+    from oracle import search_oracle as so
+    trace = {}
+    for query, q in zip(rec["queries"].tolist(), rec["query_emb"]):
+        q = q[None, :]
+        ei, es = so.similar_summaries(rec["timeline_emb"], q, rec["epi_top_k"])
+        trace[query] = _entry(rec, q, so.fact_scores(rec["fact_emb"], q), so.dense_passage_retrieval(rec["chunk_emb"], q),
+                              so.dense_passage_retrieval(rec["summary_emb"], q),
+                              ([rec["timeline_texts"][i] for i in ei.tolist()], es))
+    return {"trace": trace, "stores": {ns: rec[ns + "_keys"].tolist() for ns in STORE_NAMES}}
+
+
+class RecordedEncoder:
+    """Hands out the reference encoder's recorded rows: store texts when called without an instruction (store
+    inserts), probe rows when called with one (query encodes)."""
+    instruction_is_forced = True
+    global_config = None
+
+    def __init__(self, rec: Dict):
+        self.embedding_dim = int(rec["query_emb"].shape[1])
+        self._texts = {str(t): e for ns in STORE_NAMES for t, e in zip(rec[ns + "_texts"], rec[ns + "_emb"])}
+        self._queries = {str(t): e for t, e in zip(rec["queries"], rec["query_emb"])}
+
+    def batch_encode(self, texts, **kw) -> np.ndarray:
+        rows = self._queries if "instruction" in kw else self._texts
+        texts = [texts] if isinstance(texts, str) else texts
+        return np.stack([rows[t] for t in texts]).astype(np.float32)
+
+
+def replay_engine(rec: Dict, arm: str, workdir: str) -> Dict:
+    """The engine's side of the loop's retrieval, probe by probe, through the methods install() binds onto ComoRAG
+    (comorag_b200.comorag_methods) in tri_retrieve's order, three probes in flight as the loop's question threads do.
+    arm = "shim_search": the recorded reference rows go into engine stores (device search only);
+    arm = "shim": the engine's bf16 encoder on the synthetic checkpoint encodes the store texts and the probes.
+    Needs cuda:0.  Returns {"trace", "stores", "wave_stats", "query_encodes"}."""
+    from concurrent.futures import ThreadPoolExecutor
+    from comorag_b200 import comorag_methods as cm
+    from comorag_b200.embedding_store import EmbeddingStore
+    from comorag_b200.retrieval import get_similar_summaries
+
+    cfg = types.SimpleNamespace(embedding_model_name=CKPT, embedding_batch_size=4, embedding_max_seq_len=512,
+                                need_cluster=True, qa_epi_top_k=rec["epi_top_k"])
+    if arm == "shim":
+        from comorag_b200.embedding_model import BGEEmbeddingModel
+        model = BGEEmbeddingModel(global_config=cfg, embedding_model_name=CKPT)
+    elif arm == "shim_search":
+        model = RecordedEncoder(rec)
+    else:
+        raise ValueError(arm)
+    stores = {}
+    for ns in STORE_NAMES:
+        keys = rec[ns + "_keys"].tolist()
+        store = EmbeddingStore(model, os.path.join(workdir, ns), 4, keys[0].rsplit("-", 1)[0])
+        store.insert_strings([str(t) for t in rec[ns + "_texts"]])
+        stores[ns] = store
+    counters = {"encodes": 0, "encoded_texts": 0}
+    lock = threading.Lock()
+    orig_be = model.batch_encode
+
+    def counting_batch_encode(texts, **kw):
+        with lock:
+            counters["encodes"] += 1
+            counters["encoded_texts"] += 1 if isinstance(texts, str) else len(texts)
+        return orig_be(texts, **kw)
+    model.batch_encode = counting_batch_encode
+
+    graph = _Graph()
+    names = rec["entity_keys"].tolist() + rec["chunk_keys"].tolist()
+    graph.add_vertices(len(names), attributes={"name": names})
+    rag = types.SimpleNamespace(global_config=cfg, embedding_model=model, graph=graph, level_store=stores["timeline"],
+                                ver_embedding_store=stores["chunk"], entity_embedding_store=stores["entity"],
+                                fact_embedding_store=stores["fact"], sem_embedding_store=stores["summary"])
+    cm.prepare_retrieval_objects(rag)
+
+    def tri_retrieve(query):
+        cm.get_query_embeddings(rag, query)
+        facts = cm.get_fact_scores(rag, query)
+        ver = cm.dense_passage_retrieval(rag, query)
+        sem = cm.dense_passage_retrieval(rag, query, need_cluster=True)
+        epi = get_similar_summaries(query=query, level_store=rag.level_store, embedding_model=model,
+                                    top_k=rec["epi_top_k"])
+        return facts, ver, sem, epi
+
+    queries = rec["queries"].tolist()
+    with ThreadPoolExecutor(max_workers=3) as ex:
+        results = list(ex.map(tri_retrieve, queries))
+    wave = getattr(rag, "_crag_wave", None)
+    wave_stats = dict(wave.stats) if wave is not None else None
+    if wave is not None:
+        wave.close()
+    trace = {q: _entry(rec, q_emb, *res) for q, q_emb, res in zip(queries, rec["query_emb"], results)}
+    return {"trace": trace, "stores": {ns: s.get_all_ids() for ns, s in stores.items()}, "wave_stats": wave_stats,
+            "query_encodes": counters}

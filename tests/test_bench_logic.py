@@ -72,3 +72,12 @@ def test_both_arms_print_the_same_config_object():
         assert cfg == bench.workload_config(rows, 1024, 32, 10, world)
     src = open(bench.__file__).read()
     assert src.count('"config": workload_config(') == 2      # our arm and the reference arm, nothing hand-written beside it
+
+
+def test_dump_outputs_writes_float_arrays(tmp_path):
+    ids = np.array([[3, 1 << 40]], dtype=np.int64)
+    scores = np.array([[0.5, 0.25]], dtype=np.float32)
+    bench.dump_outputs(str(tmp_path / "out"), {"ids": ids, "scores": scores})
+    got_ids, got_scores = np.load(tmp_path / "out" / "ids.npy"), np.load(tmp_path / "out" / "scores.npy")
+    assert got_ids.dtype == np.float64 and (got_ids.astype(np.int64) == ids).all()
+    assert got_scores.dtype == np.float32 and (got_scores == scores).all()
